@@ -2,6 +2,7 @@
 """Headline benchmark of pslite_b200 (driver contract: see the task statement).
 
     python bench.py --gpus N --steps K --warmup W [--impl ours|reference] [--metric pushpull|llama|resnet]
+                    [--dump-outputs DIR]
 
 Default metric — the reference's own headline benchmark (tests/test_benchmark.cc,
 BASELINE.json "push+pull GB/s ... (test_benchmark)"): every worker ZPush-es and ZPull-s
@@ -86,7 +87,41 @@ def parse_args():
                          "the NVSwitch by the update kernel (multimem.ld_reduce)")
     ap.add_argument("--symmetric", action="store_true",
                     help="parameters in symmetric memory; NVLS multicast pull fan-out (N > 1)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what rank 0 received from the last one as DIR/<name>.npy "
+                         "(float32): pushpull the pulled values, llama / resnet the loss and the updated "
+                         "parameters. Past 60 MB in all, a fixed seeded sample of every array is written")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs records this project's timed path (--impl ours)")
+    return args
+
+
+DUMP_MAX_ELEMS = 15_000_000  # float32: 60 MB of .npy files at most
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Writes out_dir/<name>.npy (float32) for every name -> list of tensors, each list flattened and joined.
+    When all of them hold more than DUMP_MAX_ELEMS elements, every tensor keeps the same share of its
+    elements (one at least, so a loss is never dropped), at positions drawn by a generator seeded with the
+    tensor's size: the same arguments give the same positions in every run and every build."""
+    import numpy as np
+    import torch
+
+    total = sum(t.numel() for ts in arrays.values() for t in ts)
+    share = min(1.0, DUMP_MAX_ELEMS / max(total, 1))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, ts in arrays.items():
+        parts = []
+        for t in ts:
+            flat = t.detach().reshape(-1)
+            m = max(1, int(flat.numel() * share))
+            if m < flat.numel():
+                g = torch.Generator().manual_seed(flat.numel())
+                idx = torch.randint(0, flat.numel(), (m,), generator=g).sort().values
+                flat = flat[idx.to(flat.device)]
+            parts.append(flat.float().cpu())
+        np.save(os.path.join(out_dir, f"{name}.npy"), torch.cat(parts).numpy())
 
 
 # ----------------------------------------------------------------------------------------
@@ -292,6 +327,8 @@ def run_pushpull(args, dist: Dist) -> dict:
     ms, launches = timed(one_round, args.steps)
     copies_by_engine = engine_work["descriptors"]
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and dist.rank == 0:
+        dump_outputs(args.dump_outputs, {"pulled_values": vals})  # before verify() overwrites them
     verify("after the timed rounds")
     payload = float(args.len) * total_keys * W  # per step, counted once per push+pull pair
     value = payload * args.steps / (ms * 1e-3) / 1e9
@@ -498,6 +535,7 @@ def run_llama(args, dist: Dist) -> dict:
         loss = model(tok[:, :-1], tok[:, 1:])
         loss.backward()
         opt.step()
+        step.loss = loss
         return loss.item() if e2e else loss
 
     step.dev_tok = host_tok.to(dev) if ctx.is_worker else None
@@ -522,6 +560,8 @@ def run_llama(args, dist: Dist) -> dict:
     sampler = ClockSampler(dist.local_rank).start() if dist.rank == 0 and gpu.cuda else None
     ms, launches = timed(lambda: step(False), args.steps)
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and dist.rank == 0:
+        dump_outputs(args.dump_outputs, {"loss": [step.loss], "parameters": list(model.parameters())})
     tokens = B * T * W
     value = tokens * args.steps / (ms * 1e-3)
     e2e = None
@@ -590,6 +630,7 @@ def run_resnet(args, dist: Dist) -> dict:
     classes = 1000 if not tiny else 10
     model = opt = None
     if ctx.is_worker:
+        torch.manual_seed(0)  # the same initial weights in every run
         with torch.device(dev):
             model = (resnet_tiny(classes) if tiny else resnet50(classes)).to(torch.bfloat16)
         # weights and activations channels-last (cuDNN's NHWC kernels); the PS moves a weight as the flat buffer
@@ -615,6 +656,7 @@ def run_resnet(args, dist: Dist) -> dict:
         loss = loss_fn(model(img).float(), lbl)
         loss.backward()
         opt.step()
+        step.loss = loss
         return loss.item() if e2e else loss
 
     if ctx.is_worker:
@@ -640,6 +682,8 @@ def run_resnet(args, dist: Dist) -> dict:
     sampler = ClockSampler(dist.local_rank).start() if dist.rank == 0 and gpu.cuda else None
     ms, launches = timed(lambda: step(False), args.steps)
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and dist.rank == 0:
+        dump_outputs(args.dump_outputs, {"loss": [step.loss], "parameters": list(model.parameters())})
     images = B * W
     value = images * args.steps / (ms * 1e-3)
     e2e = None
@@ -752,6 +796,12 @@ def run_llama_ddp(args, dist: Dist) -> dict:
 # ----------------------------------------------------------------------------------------
 # reference arm
 # ----------------------------------------------------------------------------------------
+def reference_goodput(worker_output: str) -> float | None:
+    """Gbps of the last window the reference test_benchmark printed (the one after warm-up)."""
+    found = re.findall(r"Application goodput: ([0-9.eE+-]+) Gbps", worker_output)
+    return float(found[-1]) if found else None
+
+
 def run_reference(args, dist: Dist) -> dict:
     if args.metric != "pushpull":
         return {"impl": "reference", "unavailable":
@@ -795,9 +845,9 @@ def run_reference(args, dist: Dist) -> dict:
                 o, _ = p.communicate()
                 ok = False
             if role == "worker":
-                found = re.findall(r"Application goodput: ([0-9.eE+-]+) Gbps", o)
-                if found:
-                    gbps.append(float(found[-1]))  # last window = after warm-up
+                found = reference_goodput(o)
+                if found is not None:
+                    gbps.append(found)
                 else:
                     ok = False
         wall = time.time() - t0
