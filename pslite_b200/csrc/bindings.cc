@@ -882,13 +882,55 @@ PYBIND11_MODULE(_C, m) {
                            const std::string& optimizer, float lr, float beta1, float beta2,
                            float eps, float wd, int step, float grad_scale, int max_ctas,
                            uint64_t mc_ptr, uint64_t grad_mc_ptr) {
+    // the kernel and its CPU twin trust every size below: an undersized tensor is an out-of-bounds write
+    const int64_t n = master.numel();
+    const bool adam = optimizer == "adamw";
+    TORCH_CHECK(adam || optimizer == "sgd", "fused_update: optimizer must be 'adamw' or 'sgd'");
+    TORCH_CHECK(!adam || step >= 1, "fused_update: the AdamW step count starts at 1");
+    TORCH_CHECK(outs.size() <= PS_MAX_FANOUT, "fused_update: at most ", PS_MAX_FANOUT, " outputs");
+    auto check_tensor = [&](const torch::Tensor& t, const char* what) {
+      TORCH_CHECK(t.is_contiguous(), "fused_update: ", what, " must be contiguous");
+      TORCH_CHECK(t.device() == master.device(), "fused_update: ", what, " is on ", t.device(),
+                  ", master on ", master.device());
+    };
+    check_tensor(master, "master");
+    check_tensor(mom, "m");
+    TORCH_CHECK(mom.numel() >= n, "fused_update: m has ", mom.numel(), " elements, master ", n);
+    if (adam) {
+      check_tensor(var, "v");
+      TORCH_CHECK(var.numel() >= n, "fused_update: v has ", var.numel(), " elements, master ", n);
+    }
+    if (!grad_mc_ptr) {
+      TORCH_CHECK(grads.size() >= 1 && grads.size() <= PS_MAX_FANIN, "fused_update: 1 to ", PS_MAX_FANIN,
+                  " gradient slots, got ", grads.size());
+      const int64_t npad = (n + 31) / 32 * 32;
+      int64_t slot_bytes = 0;
+      switch (grad_format) {
+        case PS_GRAD_BF16: slot_bytes = 2 * n; break;
+        case PS_GRAD_F32: slot_bytes = 4 * n; break;
+        case PS_GRAD_FP8BLOCK: slot_bytes = npad + npad / 32; break;
+        default: TORCH_CHECK(false, "fused_update: unknown gradient format ", grad_format);
+      }
+      for (size_t i = 0; i < grads.size(); ++i) {
+        check_tensor(grads[i], "a gradient slot");
+        TORCH_CHECK(static_cast<int64_t>(grads[i].nbytes()) >= slot_bytes, "fused_update: gradient slot ", i,
+                    " holds ", grads[i].nbytes(), " bytes, the format needs ", slot_bytes);
+      }
+    }
+    for (size_t k = 0; k < outs.size(); ++k) {
+      check_tensor(outs[k], "an output");
+      TORCH_CHECK(outs[k].scalar_type() == outs[0].scalar_type() &&
+                  (outs[0].scalar_type() == torch::kBFloat16 || outs[0].scalar_type() == torch::kFloat32),
+                  "fused_update: the outputs must all be bfloat16 or all float32");
+      TORCH_CHECK(outs[k].numel() >= n, "fused_update: output ", k, " has ", outs[k].numel(),
+                  " elements, master ", n);
+    }
     ps_update_args a;
     memset(&a, 0, sizeof(a));
-    a.n = static_cast<size_t>(master.numel());
+    a.n = static_cast<size_t>(n);
     a.num_grads = static_cast<int>(grads.size());
     a.grad_format = grad_format;
-    TORCH_CHECK(a.num_grads <= PS_MAX_FANIN && outs.size() <= PS_MAX_FANOUT);
-    for (size_t i = 0; i < grads.size(); ++i) a.grads[i] = grads[i].data_ptr();
+    for (size_t i = 0; i < grads.size() && i < PS_MAX_FANIN; ++i) a.grads[i] = grads[i].data_ptr();
     if (grad_mc_ptr) {  // PS_GRAD_MC_BF16: the gradients are read through a multicast address
       a.num_grads = 1;
       a.grads[0] = reinterpret_cast<const void*>(grad_mc_ptr);

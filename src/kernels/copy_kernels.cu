@@ -32,12 +32,19 @@ std::atomic<unsigned long long> g_launches{0};
 
 constexpr int kThreads = 256;
 
-/*! \brief SM count of the current device (148 on B200), asked once per device */
-int NumSMs() {
-  static std::atomic<int> cached[16] = {};
+constexpr int kMaxDevices = 16;
+
+/*! \brief index of the current device for per-device caches, in [0, kMaxDevices) */
+int CurrentDevice() {
   int dev = 0;
   cudaGetDevice(&dev);
-  if (dev < 0 || dev >= 16) dev = 0;
+  return dev < 0 || dev >= kMaxDevices ? 0 : dev;
+}
+
+/*! \brief SM count of the current device (148 on B200), asked once per device */
+int NumSMs() {
+  static std::atomic<int> cached[kMaxDevices] = {};
+  const int dev = CurrentDevice();
   int n = cached[dev].load(std::memory_order_relaxed);
   if (n == 0) {
     if (cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || n <= 0) n = 148;
@@ -340,14 +347,18 @@ __global__ void k_bf16_scale_tail(__nv_bfloat16* dst, const __nv_bfloat16* src, 
 // ---------------------------------------------------------------------------
 // block-scaled fp8 (e4m3 payload, one e8m0 exponent per 32 elements)
 // ---------------------------------------------------------------------------
-/*! exponent e such that amax / 2^e <= 448 (largest finite e4m3); biased by 127 */
+/*!
+ * exponent e such that amax / 2^e <= 448 (largest finite e4m3); biased by 127. e is clamped to
+ * [-126, 127]: the decoders read byte 0 as 2^-126 (the smallest normal fp32 scale), so byte 0 is
+ * left to the all-zero block, where any scale decodes to zero.
+ */
 __device__ __forceinline__ uint32_t e8m0_for_amax(float amax) {
   if (!(amax > 0.f)) return 0u;
   const uint32_t bits = __float_as_uint(amax);
   int k = static_cast<int>((bits >> 23) & 0xff) - 127;     // amax = m * 2^k, m in [1,2)
   const uint32_t mant = bits & 0x7fffffu;
   int e = k - 8 + (mant > 0x600000u ? 1 : 0);              // 448 = 1.75 * 2^8
-  e = max(-127, min(127, e));
+  e = max(-126, min(127, e));
   return static_cast<uint32_t>(e + 127);
 }
 __device__ __forceinline__ float exp2_from_e8m0_neg(uint32_t biased) {
@@ -497,6 +508,7 @@ extern "C" unsigned long long ps_kernel_launch_count(void) { return g_launches.l
 namespace ps_kernels_internal {
 void CountLaunch(int n) { g_launches += static_cast<unsigned long long>(n); }
 int NumSMs() { return ::NumSMs(); }
+int CurrentDevice() { return ::CurrentDevice(); }
 }
 
 extern "C" int ps_launch_signal(const ps_signal* sig, ps_stream_t stream_) {
@@ -530,11 +542,12 @@ extern "C" int ps_launch_copy_signal(void* dst, const void* src, size_t n, int c
         break;
       }
       if (UseTma() && n >= static_cast<size_t>(kTmaChunk)) {
-        static std::atomic<bool> attr_set{false};
+        static std::atomic<bool> attr_set[kMaxDevices] = {};  // the attribute is per device
         const int smem_bytes = kTmaStages * kTmaChunk;
-        if (!attr_set.load(std::memory_order_acquire)) {
+        const int dev = CurrentDevice();
+        if (!attr_set[dev].load(std::memory_order_acquire)) {
           cudaFuncSetAttribute(k_copy_tma, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes);
-          attr_set.store(true, std::memory_order_release);
+          attr_set[dev].store(true, std::memory_order_release);
         }
         const size_t body = n & ~size_t(15);
         const size_t chunks = (body + kTmaChunk - 1) / kTmaChunk;

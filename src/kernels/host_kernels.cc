@@ -86,7 +86,7 @@ inline uint32_t E8m0ForAmax(float amax) {
   const int k = static_cast<int>((bits >> 23) & 0xff) - 127;
   const uint32_t mant = bits & 0x7fffffu;
   int e = k - 8 + (mant > 0x600000u ? 1 : 0);  // 448 = 1.75 * 2^8
-  e = std::max(-127, std::min(127, e));
+  e = std::max(-126, std::min(127, e));         // byte 0 only for the all-zero block (see copy_kernels.cu)
   return static_cast<uint32_t>(e + 127);
 }
 inline float Exp2FromE8m0(uint32_t biased) {

@@ -40,7 +40,9 @@ enum {
 enum {
   PS_GRAD_F32 = 0,
   PS_GRAD_BF16 = 1,
-  PS_GRAD_FP8BLOCK = 2,  // [n_pad e4m3 bytes][n_pad/32 e8m0 bytes], n_pad = roundup(n,32)
+  /* [n_pad e4m3 bytes][n_pad/32 e8m0 bytes], n_pad = roundup(n,32). Scale byte b means 2^(b-127);
+   * encoders write b in [1, 254] (exponent in [-126, 127]) and b = 0 only for an all-zero block. */
+  PS_GRAD_FP8BLOCK = 2,
   /* NVLS in-switch aggregation: grads[0] is a MULTICAST address bound to the same offset of
    * every worker's (symmetric) bf16 gradient buffer; num_grads must be 1. The kernel reads it
    * with multimem.ld_reduce.add (fp32 accumulation inside the NVSwitch), so the W-way sum
@@ -155,7 +157,11 @@ typedef struct {
   int body_outs;
 } ps_update_args;
 
-/*! \brief fused dequant + W-way sum + optimizer + bf16 fan-out for one shard */
+/*!
+ * \brief fused dequant + W-way sum + optimizer + bf16 fan-out for one shard
+ * \return cudaErrorMisalignedAddress, before anything is launched, unless master, m, v (AdamW),
+ *         every grads[w], every outs[k] and mc_out are 16-byte aligned
+ */
 int ps_launch_update(const ps_update_args* args, const ps_opt_params* opt, int max_ctas,
                      ps_stream_t stream);
 

@@ -33,11 +33,13 @@
 namespace ps_kernels_internal {
 void CountLaunch(int n);
 int NumSMs();
+int CurrentDevice();
 }
 
 namespace {
 
 constexpr int kThreads = 256;
+constexpr int kMaxDevices = 16;  // as in NumSMs(): per-device caches (CurrentDevice() maps others to 0)
 
 struct UpdateDev {
   size_t n;
@@ -501,18 +503,14 @@ bool LaunchUpdateTmaImpl(const UpdateDev& d, const ps_opt_params& o, bool out_f3
   const int stage = 3 * kTile * 4 + d.num_grads * GradTileBytes<FMT>();
   const int smem = kTmaStagesU * stage;
   if (tiles < 4 || smem > 220 * 1024) return false;
-  // cp.async.bulk needs 16-byte aligned sources (landing slots are 512-byte aligned, state is cudaMalloc'ed)
-  if ((reinterpret_cast<uintptr_t>(d.master) | reinterpret_cast<uintptr_t>(d.m) |
-       reinterpret_cast<uintptr_t>(d.v)) & 15) {
-    return false;
-  }
-  for (int w = 0; w < d.num_grads; ++w) {
-    if (reinterpret_cast<uintptr_t>(d.grads[w]) & 15) return false;
-  }
-  static std::atomic<bool> attr_set{false};  // (one per instantiation; launches come from several threads)
-  if (!attr_set.load(std::memory_order_acquire)) {
+  // (cp.async.bulk needs 16-byte aligned sources: ps_launch_update has refused anything else)
+  // the attribute belongs to the current device: one flag per device and instantiation
+  // (launches come from several threads, and a process may drive several GPUs)
+  static std::atomic<bool> attr_set[kMaxDevices] = {};
+  const int dev = ps_kernels_internal::CurrentDevice();
+  if (!attr_set[dev].load(std::memory_order_acquire)) {
     cudaFuncSetAttribute(k_update_tma<FMT, OPT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024);
-    attr_set.store(true, std::memory_order_release);
+    attr_set[dev].store(true, std::memory_order_release);
   }
   const int num_sms = ps_kernels_internal::NumSMs();
   int grid = static_cast<int>(tiles < static_cast<size_t>(num_sms) ? tiles : num_sms);
@@ -559,6 +557,13 @@ extern "C" int ps_launch_update(const ps_update_args* args, const ps_opt_params*
   d.mc_out = args->out_f32 ? nullptr : args->mc_out;
   d.body_outs = d.mc_out ? args->body_outs : args->num_outs;
   if (d.body_outs < 0 || d.body_outs > args->num_outs) return cudaErrorInvalidValue;
+  // both flavours move 16-byte vectors (ld/st.v4, cp.async.bulk) through every one of these pointers
+  uintptr_t addr_bits = reinterpret_cast<uintptr_t>(d.master) | reinterpret_cast<uintptr_t>(d.m) |
+                        reinterpret_cast<uintptr_t>(d.mc_out);
+  if (opt->optimizer == PS_OPT_ADAMW) addr_bits |= reinterpret_cast<uintptr_t>(d.v);
+  for (int w = 0; w < d.num_grads; ++w) addr_bits |= reinterpret_cast<uintptr_t>(d.grads[w]);
+  for (int k = 0; k < d.num_outs; ++k) addr_bits |= reinterpret_cast<uintptr_t>(d.outs[k]);
+  if (addr_bits & 15) return cudaErrorMisalignedAddress;
   // 2 resident CTAs/SM x 148 keeps ~100 KB of loads in flight per SM
   const int grid = GridFor(args->n / 8 + 1, max_ctas, 4);
   const bool f32 = args->out_f32 != 0;

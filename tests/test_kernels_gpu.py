@@ -16,7 +16,7 @@ def ref_fp8_block(x: torch.Tensor):
     pad = (32 - n % 32) % 32
     xp = torch.cat([x.float(), x.new_zeros(pad, dtype=torch.float32)]).view(-1, 32)
     amax = xp.abs().amax(dim=1)
-    e = torch.ceil(torch.log2(amax.clamp_min(1e-38) / 448.0)).clamp(-127, 127)
+    e = torch.ceil(torch.log2(amax.clamp_min(1e-38) / 448.0)).clamp(-126, 127)  # 2^-126: smallest decodable scale
     e = torch.where(amax > 0, e, torch.full_like(e, -127.0))
     scale = torch.exp2(e)
     q = (xp / scale[:, None]).to(torch.float8_e4m3fn).float() * scale[:, None]

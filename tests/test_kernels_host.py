@@ -139,9 +139,12 @@ def test_host_fused_sgd_update(native):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("codec_name", ["CODEC_F32_TO_BF16", "CODEC_F32_TO_FP8BLOCK", "CODEC_BF16_TO_FP8BLOCK"])
+@pytest.mark.parametrize("codec_name", ["CODEC_F32_TO_BF16", "CODEC_BF16_SCALE", "CODEC_F32_TO_FP8BLOCK",
+                                        "CODEC_BF16_TO_FP8BLOCK"])
 def test_gpu_wire_bytes_equal_host_wire_bytes(native, codec_name):
-    """the sm_100a push kernels and their CPU twins produce the same bytes for the same input"""
+    """the sm_100a push kernels and their CPU twins produce the same bytes for the same input, also
+    from and to views that are not 16-byte aligned (the bf16 codecs then run their scalar tail
+    kernel; the fp8 codec refuses a misaligned source before launching anything)"""
     if not torch.cuda.is_available():
         pytest.skip("no CUDA device")
     codec = getattr(native, codec_name)
@@ -156,3 +159,18 @@ def test_gpu_wire_bytes_equal_host_wire_bytes(native, codec_name):
     native.copy_codec(dev, x.cuda().view(torch.uint8), codec, 0.5)
     torch.cuda.synchronize()
     assert torch.equal(dev.cpu(), host)
+
+    # the same input one element into a larger buffer: 4 (f32) or 2 (bf16) bytes off 16-byte alignment
+    src_shifted = torch.zeros(n + 1, dtype=x.dtype, device="cuda")
+    src_shifted[1:] = x.cuda()
+    src_shifted = src_shifted[1:]
+    if codec_name.endswith("FP8BLOCK"):
+        with pytest.raises(RuntimeError, match="misaligned"):
+            native.copy_codec(dev, src_shifted.view(torch.uint8), codec, 0.5)
+        return
+    for src, dst_off in ((src_shifted, 0), (x.cuda(), 2), (src_shifted, 2)):
+        out = torch.full((nbytes + dst_off,), 0xA5, dtype=torch.uint8, device="cuda")
+        native.copy_codec(out[dst_off:], src.view(torch.uint8), codec, 0.5)
+        torch.cuda.synchronize()
+        assert torch.equal(out[dst_off:].cpu(), host), f"source shifted: {src is src_shifted}, destination +{dst_off}"
+        assert bool((out[:dst_off] == 0xA5).all())
