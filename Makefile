@@ -38,7 +38,7 @@ CU_SRCS :=
 ifeq ($(USE_CUDA),1)
 CXXFLAGS += -DPS_USE_CUDA=1 -I$(CUDA_HOME)/include
 CORE_SRCS += src/van/cuda_domain.cc src/van/nccl_van.cc
-CU_SRCS += src/kernels/copy_kernels.cu src/kernels/update_kernels.cu src/kernels/model_kernels.cu src/kernels/engine_kernels.cu
+CU_SRCS += src/kernels/copy_kernels.cu src/kernels/update_kernels.cu src/kernels/update_rows_kernels.cu src/kernels/model_kernels.cu src/kernels/engine_kernels.cu
 LDFLAGS += -L$(CUDA_HOME)/lib64 -lcudart -ldl
 endif
 

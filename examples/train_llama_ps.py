@@ -33,6 +33,8 @@ def main():
     ap.add_argument("--lr", type=float, default=3e-4)
     ap.add_argument("--grad-wire", default="fp8", choices=["fp8", "bf16"])
     ap.add_argument("--fused-pushpull", action="store_true")
+    ap.add_argument("--sparse-embedding", action="store_true",
+                    help="row-sparse input embedding: push only the rows a batch touched")
     args = ap.parse_args()
 
     use_cuda = torch.cuda.is_available()
@@ -48,12 +50,13 @@ def main():
     server = C.GpuServer(0, num_workers=ctx.num_workers, optimizer="adamw", lr=args.lr,
                          grad_scale=1.0 / ctx.num_workers)
 
+    sparse = dict(sparse_embedding=args.sparse_embedding)
     if args.model == "tiny":
-        cfg = LlamaConfig.tiny()
+        cfg = LlamaConfig.tiny(**sparse)
     elif args.model == "llama-1b":
-        cfg = LlamaConfig(dim=2048, n_layers=16, n_heads=32, n_kv_heads=8, ffn_dim=8192, ckpt_layers=0)
+        cfg = LlamaConfig(dim=2048, n_layers=16, n_heads=32, n_kv_heads=8, ffn_dim=8192, ckpt_layers=0, **sparse)
     else:
-        cfg = LlamaConfig.llama3_8b(ckpt_layers=0)
+        cfg = LlamaConfig.llama3_8b(ckpt_layers=0, **sparse)
     seq = args.seq_len or min(cfg.max_seq_len, 8192 if args.model != "tiny" else 64)
     with torch.device(dev):
         model = Llama(cfg).to(torch.bfloat16)
@@ -61,17 +64,27 @@ def main():
 
     kv = C.KVWorker(0, 0)
     opt = PSWorkerOptimizer(model.parameters(), kv, ctx.num_servers, ctx.num_workers, ctx.worker_rank,
-                            grad_wire=args.grad_wire, fused_pushpull=args.fused_pushpull).attach()
+                            grad_wire=args.grad_wire, fused_pushpull=args.fused_pushpull,
+                            row_sparse=[model.embed.weight] if args.sparse_embedding else ()).attach()
     opt.init_parameters(barrier=lambda: C.barrier(0, C.WORKER_GROUP, "worker"))
 
     g = torch.Generator(device=dev).manual_seed(1 + ctx.worker_rank)
     tok = torch.randint(0, cfg.vocab_size, (1, seq + 1), device=dev, generator=g)
+    import time
+
+    times, wire = [], []
     for step in range(args.steps):
+        t0, b0 = time.perf_counter(), opt.stats.push_bytes_wire
         loss = model(tok[:, :-1], tok[:, 1:])
         loss.backward()   # gradients are pushed from the hooks while backward still runs
         opt.step()        # every parameter chunk has been rewritten by its server
+        if use_cuda:
+            torch.cuda.synchronize()
+        times.append(time.perf_counter() - t0)
+        wire.append(opt.stats.push_bytes_wire - b0)
         if ctx.worker_rank == 0:
-            print(f"step {step}: loss {loss.item():.4f}", flush=True)
+            print(f"step {step}: loss {loss.item():.4f} time {times[-1] * 1e3:.1f} ms "
+                  f"push_bytes_wire {wire[-1]}", flush=True)
     if ctx.worker_rank == 0:
         print(f"server 0: {server.num_updates()} updates on the {'device' if server.on_device() else 'host'} engine")
     ctx.shutdown()

@@ -303,6 +303,13 @@ struct SendOpts {
   MemRef pull_dest_mem;
   /*! \brief value of Meta::option / KVMeta::option (application-defined flags) */
   int option = 0;
+  /*!
+   * \brief push over a one-sided van: request the landing slot at this capacity and reuse it for
+   *        every push of the key that fits, however much smaller (pushes whose size changes every
+   *        step, e.g. row-sparse gradients). 0: the slot is re-made when a push outgrows it or
+   *        shrinks far below it.
+   */
+  uint64_t slot_bytes = 0;
 };
 
 /*! \brief MemRef::region value meaning "offset inside the job-wide symmetric buffer" */
@@ -316,6 +323,8 @@ struct Message {
   void* wait_event = nullptr;
   /*! \brief local-only: staging address of a symmetric push (see SendOpts::stage) */
   void* stage = nullptr;
+  /*! \brief local-only: landing-slot capacity to request (see SendOpts::slot_bytes) */
+  uint64_t slot_bytes = 0;
 
   /*! \brief append a segment; the second one (the values) sets the placement fields */
   template <typename V>

@@ -545,6 +545,7 @@ void KVWorker<Val>::Send(int timestamp, bool push, int cmd, KVPairs<Val>& kvs,
     msg.meta.scale = opts.scale;
     msg.meta.option = opts.option;
     msg.wait_event = opts.wait_event;
+    msg.slot_bytes = opts.slot_bytes;
     if (opts.dest_mem.valid()) {
       msg.meta.mem = opts.dest_mem;
       if (push) msg.stage = opts.stage;

@@ -92,12 +92,14 @@ class PyKVWorker {
   }
 
   int push(uint64_t key, const torch::Tensor& t, int cmd, int codec, float scale,
-           bool order_after_current_stream, int64_t symm_offset, uint64_t symm_base, int option) {
+           bool order_after_current_stream, int64_t symm_offset, uint64_t symm_base, int option,
+           uint64_t slot_bytes) {
     SArray<char> vals = ViewOf(t);
     SendOpts opts;
     opts.codec = codec;
     opts.scale = scale;
     opts.option = option;
+    opts.slot_bytes = slot_bytes;
     if (symm_offset >= 0) {
       // stage the encoded gradient in this worker's symmetric buffer; the server reads the
       // sum of all workers' copies through the multicast address (multimem.ld_reduce)
@@ -527,6 +529,10 @@ class PyGpuServer {
   uint64_t num_fused_fanouts() { return impl_->num_fused_fanouts(); }
   size_t num_keys() { return impl_->num_keys(); }
   size_t state_bytes() { return impl_->state_bytes(); }
+  uint64_t num_bad_rows() {
+    py::gil_scoped_release nogil;
+    return impl_->num_bad_rows();
+  }
   bool save(const std::string& path) {
     py::gil_scoped_release nogil;
     return impl_->SaveCheckpoint(path);
@@ -551,6 +557,16 @@ ps_stream_t CurrentStream(const torch::Tensor& t) {
 
 void CheckRc(int rc, const char* what) {
   TORCH_CHECK(rc == 0, what, " failed: ", cudaGetErrorString(static_cast<cudaError_t>(rc)));
+}
+
+/*! \brief bytes of a row-sparse gradient slot (ps_update_rows_args): ids padded to 16 B, then the values */
+int64_t RowsSlotBytes(int64_t num_rows, int64_t dim, int grad_format) {
+  const int64_t ids = (num_rows + 3) / 4 * 16, e = num_rows * dim;
+  switch (grad_format) {
+    case PS_GRAD_F32: return ids + 4 * e;
+    case PS_GRAD_BF16: return ids + 2 * e;
+    default: return ids + e + e / 32;  // fp8 block: dim % 32 == 0
+  }
 }
 
 }  // namespace
@@ -594,6 +610,8 @@ PYBIND11_MODULE(_C, m) {
   m.attr("GRAD_BF16") = static_cast<int>(PS_GRAD_BF16);
   m.attr("CMD_SET_LR") = static_cast<int>(kCmdSetLr);
   m.attr("INIT_NO_WEIGHT_DECAY") = static_cast<int>(kInitNoWeightDecay);
+  m.attr("INIT_ROW_SPARSE") = static_cast<int>(kInitRowSparse);
+  m.attr("CMD_GRAD_ROWS") = static_cast<int>(kCmdGradRows);
   m.attr("GRAD_FP8BLOCK") = static_cast<int>(PS_GRAD_FP8BLOCK);
   m.attr("GRAD_MC_BF16") = static_cast<int>(PS_GRAD_MC_BF16);
 
@@ -704,7 +722,7 @@ PYBIND11_MODULE(_C, m) {
       .def("push", &PyKVWorker::push, py::arg("key"), py::arg("tensor"), py::arg("cmd") = 0,
            py::arg("codec") = 0, py::arg("scale") = 1.0f,
            py::arg("order_after_current_stream") = true, py::arg("symm_offset") = -1,
-           py::arg("symm_base") = 0, py::arg("option") = 0)
+           py::arg("symm_base") = 0, py::arg("option") = 0, py::arg("slot_bytes") = 0)
       .def("pull", &PyKVWorker::pull, py::arg("key"), py::arg("tensor"), py::arg("cmd") = 0,
            py::arg("symm_offset") = -1)
       .def("push_pull", &PyKVWorker::push_pull, py::arg("key"), py::arg("tensor"), py::arg("out"),
@@ -758,6 +776,7 @@ PYBIND11_MODULE(_C, m) {
       .def("num_fused_fanouts", &PyGpuServer::num_fused_fanouts)
       .def("num_keys", &PyGpuServer::num_keys)
       .def("state_bytes", &PyGpuServer::state_bytes)
+      .def("num_bad_rows", &PyGpuServer::num_bad_rows)
       .def("save", &PyGpuServer::save)
       .def("load", &PyGpuServer::load)
       .def("read_master", &PyGpuServer::read_master);
@@ -959,4 +978,100 @@ PYBIND11_MODULE(_C, m) {
      py::arg("beta1") = 0.9f, py::arg("beta2") = 0.95f, py::arg("eps") = 1e-8f,
      py::arg("weight_decay") = 0.0f, py::arg("step") = 1, py::arg("grad_scale") = 1.0f,
      py::arg("max_ctas") = 0, py::arg("mc_ptr") = 0, py::arg("grad_mc_ptr") = 0);
+  m.def("rows_scratch_bytes", [](uint64_t rows, int max_grads) {
+    return static_cast<uint64_t>(ps_rows_scratch_bytes(rows, max_grads));
+  });
+  m.def("rows_slot_bytes", [](int64_t num_rows, int64_t dim, int grad_format) {
+    return RowsSlotBytes(num_rows, dim, grad_format);
+  });
+  m.def("fused_update_rows", [](std::vector<torch::Tensor> grads, std::vector<int64_t> num_rows, int grad_format,
+                                int64_t dim, torch::Tensor master, torch::Tensor mom, torch::Tensor var,
+                                std::vector<torch::Tensor> outs, torch::Tensor scratch,
+                                const std::string& optimizer, float lr, float beta1, float beta2, float eps,
+                                float wd, int step, float grad_scale, int max_ctas) {
+    // the kernel and its CPU twin trust every size below: an undersized tensor is an out-of-bounds access
+    const int64_t n = master.numel();
+    const bool adam = optimizer == "adamw";
+    TORCH_CHECK(adam || optimizer == "sgd", "fused_update_rows: optimizer must be 'adamw' or 'sgd'");
+    TORCH_CHECK(!adam || step >= 1, "fused_update_rows: the AdamW step count starts at 1");
+    TORCH_CHECK(grads.size() >= 1 && grads.size() <= PS_MAX_FANIN, "fused_update_rows: 1 to ", PS_MAX_FANIN,
+                " gradient slots, got ", grads.size());
+    TORCH_CHECK(num_rows.size() == grads.size(), "fused_update_rows: ", grads.size(), " slots but ",
+                num_rows.size(), " row counts");
+    TORCH_CHECK(outs.size() <= PS_MAX_FANOUT, "fused_update_rows: at most ", PS_MAX_FANOUT, " outputs");
+    TORCH_CHECK(grad_format == PS_GRAD_F32 || grad_format == PS_GRAD_BF16 || grad_format == PS_GRAD_FP8BLOCK,
+                "fused_update_rows: unknown gradient format ", grad_format);
+    TORCH_CHECK(dim > 0 && dim % 8 == 0, "fused_update_rows: the row width must be a positive multiple of 8, got ",
+                dim);
+    TORCH_CHECK(grad_format != PS_GRAD_FP8BLOCK || dim % 32 == 0,
+                "fused_update_rows: fp8 rows need a row width that is a multiple of 32, got ", dim);
+    TORCH_CHECK(master.scalar_type() == torch::kFloat32 && n % dim == 0,
+                "fused_update_rows: master must be float32 with a whole number of rows of ", dim);
+    const int64_t rows = n / dim;
+    auto check_tensor = [&](const torch::Tensor& t, const char* what) {
+      TORCH_CHECK(t.is_contiguous(), "fused_update_rows: ", what, " must be contiguous");
+      TORCH_CHECK(t.device() == master.device(), "fused_update_rows: ", what, " is on ", t.device(),
+                  ", master on ", master.device());
+    };
+    check_tensor(master, "master");
+    check_tensor(mom, "m");
+    TORCH_CHECK(mom.scalar_type() == torch::kFloat32 && mom.numel() >= n, "fused_update_rows: m must be float32 with ",
+                n, " elements");
+    if (adam) {
+      check_tensor(var, "v");
+      TORCH_CHECK(var.scalar_type() == torch::kFloat32 && var.numel() >= n,
+                  "fused_update_rows: v must be float32 with ", n, " elements");
+    }
+    for (size_t i = 0; i < grads.size(); ++i) {
+      check_tensor(grads[i], "a gradient slot");
+      TORCH_CHECK(num_rows[i] >= 0 && num_rows[i] <= 0xffffffffll, "fused_update_rows: bad row count ",
+                  num_rows[i]);
+      const int64_t need = RowsSlotBytes(num_rows[i], dim, grad_format);
+      TORCH_CHECK(static_cast<int64_t>(grads[i].nbytes()) >= need, "fused_update_rows: gradient slot ", i, " holds ",
+                  grads[i].nbytes(), " bytes, ", num_rows[i], " rows need ", need);
+    }
+    for (size_t k = 0; k < outs.size(); ++k) {
+      check_tensor(outs[k], "an output");
+      TORCH_CHECK(outs[k].scalar_type() == outs[0].scalar_type() &&
+                  (outs[0].scalar_type() == torch::kBFloat16 || outs[0].scalar_type() == torch::kFloat32),
+                  "fused_update_rows: the outputs must all be bfloat16 or all float32");
+      TORCH_CHECK(outs[k].numel() >= n, "fused_update_rows: output ", k, " has ", outs[k].numel(),
+                  " elements, master ", n);
+    }
+    check_tensor(scratch, "scratch");
+    const size_t scratch_need = ps_rows_scratch_bytes(static_cast<size_t>(rows), static_cast<int>(grads.size()));
+    TORCH_CHECK(scratch.nbytes() >= scratch_need, "fused_update_rows: scratch holds ", scratch.nbytes(),
+                " bytes, needs ", scratch_need);
+    ps_update_rows_args a;
+    memset(&a, 0, sizeof(a));
+    a.rows = static_cast<size_t>(rows);
+    a.dim = static_cast<int>(dim);
+    a.num_grads = static_cast<int>(grads.size());
+    a.grad_format = grad_format;
+    for (size_t i = 0; i < grads.size(); ++i) {
+      a.grads[i] = grads[i].data_ptr();
+      a.num_rows[i] = static_cast<uint32_t>(num_rows[i]);
+    }
+    a.master = master.data_ptr<float>();
+    a.m = mom.data_ptr<float>();
+    a.v = adam ? var.data_ptr<float>() : nullptr;
+    a.num_outs = static_cast<int>(outs.size());
+    for (size_t i = 0; i < outs.size(); ++i) a.outs[i] = outs[i].data_ptr();
+    a.out_f32 = !outs.empty() && outs[0].scalar_type() == torch::kFloat32;
+    a.scratch = scratch.data_ptr();
+    ps_opt_params o;
+    o.optimizer = adam ? PS_OPT_ADAMW : PS_OPT_SGD;
+    o.lr = lr; o.beta1 = beta1; o.beta2 = beta2; o.eps = eps; o.weight_decay = wd;
+    o.bias_corr1 = adam ? 1.f - std::pow(beta1, (float)step) : 1.f;
+    o.bias_corr2 = adam ? 1.f - std::pow(beta2, (float)step) : 1.f;
+    o.grad_scale = grad_scale;
+    if (!master.is_cuda()) {
+      TORCH_CHECK(ps_host_update_rows(&a, &o) == 0, "ps_host_update_rows: bad arguments");
+      return;
+    }
+    CheckRc(ps_launch_update_rows(&a, &o, max_ctas, CurrentStream(master)), "ps_launch_update_rows");
+  }, py::arg("grads"), py::arg("num_rows"), py::arg("grad_format"), py::arg("dim"), py::arg("master"),
+     py::arg("m"), py::arg("v"), py::arg("outs"), py::arg("scratch"), py::arg("optimizer") = "adamw",
+     py::arg("lr") = 1e-3f, py::arg("beta1") = 0.9f, py::arg("beta2") = 0.95f, py::arg("eps") = 1e-8f,
+     py::arg("weight_decay") = 0.0f, py::arg("step") = 1, py::arg("grad_scale") = 1.0f, py::arg("max_ctas") = 0);
 }

@@ -35,6 +35,7 @@ class LlamaConfig:
     loss_chunk: int = 2048         # tokens per LM-head / cross-entropy chunk
     attn_backend: str = "auto"     # auto | cudnn | flash | efficient | math (PyTorch SDPA backends)
     fused_ops: bool = True         # own RoPE-split / SwiGLU kernels on CUDA (pslite_b200.ops.fused)
+    sparse_embedding: bool = False # input embedding with sparse (row) gradients: nn.Embedding(sparse=True)
 
     @staticmethod
     def llama3_8b(**kw) -> "LlamaConfig":
@@ -165,7 +166,7 @@ class Llama(nn.Module):
     def __init__(self, cfg: LlamaConfig):
         super().__init__()
         self.cfg = cfg
-        self.embed = nn.Embedding(cfg.vocab_size, cfg.dim)
+        self.embed = nn.Embedding(cfg.vocab_size, cfg.dim, sparse=cfg.sparse_embedding)
         self.layers = nn.ModuleList(Block(cfg) for _ in range(cfg.n_layers))
         self.norm = RMSNorm(cfg.dim, cfg.norm_eps)
         self.lm_head = nn.Linear(cfg.dim, cfg.vocab_size, bias=False)

@@ -17,6 +17,11 @@ Worker side of the BytePS-style loop the reference is built for (docs/overview.m
 
 The optimizer state (fp32 master, Adam moments) lives only on the servers, sharded by key.
 
+Embedding tables whose gradients are sparse (`nn.Embedding(sparse=True)`) can be passed as
+`row_sparse`: they are chunked on row boundaries, each worker pushes only the rows its batch
+touched (ids + values, `CMD_GRAD_ROWS`), and the server steps and rewrites only the union of
+those rows ("lazy" AdamW / SGD: untouched rows get no momentum step and no weight decay).
+
 With NVSwitch multicast (`symmetric=True`, `grad_buffer=...`) a whole round is ONE kernel per
 shard that never touches NCCL: `multimem.ld_reduce` (the switch sums the W workers' gradient
 buffers in fp32) -> AdamW on the fp32 state -> `multimem.st` (the switch replicates the new
@@ -39,6 +44,7 @@ class _Chunk:
     start: int
     stop: int
     server: int
+    dim: int = 0  # row-sparse parameter: row width (the chunk is whole rows); 0 = dense
 
 
 @dataclass
@@ -147,7 +153,7 @@ class PSWorkerOptimizer:
     def __init__(self, params, kv, num_servers: int, num_workers: int, worker_rank: int,
                  grad_wire: str = "fp8", chunk_elems: int = 32 << 20, app_barrier=None,
                  symmetric: bool = False, grad_buffer: torch.Tensor | None = None,
-                 fused_pushpull: bool = False, no_decay_1d: bool = True):
+                 fused_pushpull: bool = False, no_decay_1d: bool = True, row_sparse=()):
         C = native()
         self._C = C
         self.kv = kv
@@ -176,6 +182,10 @@ class PSWorkerOptimizer:
         self.no_decay_1d = no_decay_1d
         assert not (fused_pushpull and grad_buffer is not None), "push-pull stages no symmetric gradients"
         self.grad_buffer = grad_buffer
+        # 2-D parameters whose gradients arrive as sparse COO tensors (nn.Embedding(sparse=True))
+        self.row_sparse = {id(p) for p in row_sparse}
+        assert not (self.row_sparse and grad_buffer is not None), "row-sparse gradients are not reduced in the switch"
+        self._staging: dict[int, torch.Tensor] = {}  # key -> worst-case row push of that chunk
         if grad_buffer is not None:
             assert symmetric, "in-switch reduction uses the symmetric parameter layout"
             assert grad_buffer.dtype == torch.bfloat16 and grad_buffer.is_contiguous()
@@ -186,12 +196,20 @@ class PSWorkerOptimizer:
             _flat(p.data)  # (asserts that the parameter is dense)
             per = []
             n = p.numel()
-            for a in range(0, n, chunk_elems):
-                b = min(n, a + chunk_elems)
+            dim = 0
+            step = chunk_elems
+            if id(p) in self.row_sparse:
+                assert p.dim() == 2, "row_sparse parameters are 2-D tables"
+                dim = p.shape[1]
+                step = max(1, chunk_elems // dim) * dim  # whole rows per key
+            for a in range(0, n, step):
+                b = min(n, a + step)
                 server = j % self.S
-                per.append(_Chunk(kv.server_key(server, j), i, a, b, server))
+                per.append(_Chunk(kv.server_key(server, j), i, a, b, server, dim))
                 j += 1
             self.chunks.append(per)
+        assert len(self.row_sparse) == sum(1 for per in self.chunks if per and per[0].dim), \
+            "every row_sparse parameter must be one of the trained parameters"
         self.stats.keys = j
 
     # -- wire format -------------------------------------------------------------
@@ -216,7 +234,8 @@ class PSWorkerOptimizer:
                 cmd = C.CMD_INIT_F32 if p.dtype == torch.float32 else C.CMD_INIT_BF16
                 opt_bits = C.INIT_NO_WEIGHT_DECAY if (self.no_decay_1d and p.dim() <= 1) else 0
                 for c in per:
-                    ts.append(self.kv.push(c.key, flat[c.start:c.stop], cmd=cmd, option=opt_bits))
+                    bits = opt_bits | (C.INIT_ROW_SPARSE | (c.dim << 8) if c.dim else 0)
+                    ts.append(self.kv.push(c.key, flat[c.start:c.stop], cmd=cmd, option=bits))
             for t in ts:
                 self.kv.wait(t)
         (barrier or self._barrier or (lambda: None))()
@@ -290,7 +309,60 @@ class PSWorkerOptimizer:
             return
         self._push_pull_now(i, g)
 
+    def _row_format(self, dim: int) -> int:
+        C = self._C
+        return C.GRAD_FP8BLOCK if self.grad_wire == "fp8" and dim % 32 == 0 else C.GRAD_BF16
+
+    def _push_rows(self, i: int, g: torch.Tensor):
+        """push the touched rows of every chunk of a row-sparse parameter, then pull the chunk"""
+        C = self._C
+        p = self.params[i].data
+        if not g.is_sparse:
+            raise ValueError(f"parameter {i} is row_sparse but its gradient is dense: build it with "
+                             "nn.Embedding(sparse=True) or leave it out of row_sparse")
+        g = g.float().coalesce()  # (repeated tokens of a batch are summed in fp32, not in the gradient's bf16)
+        ids = g.indices()[0]
+        vals = g.values()
+        per = self.chunks[i]
+        dim = per[0].dim
+        fmt = self._row_format(dim)
+        bounds = torch.tensor([c.start // dim for c in per] + [per[-1].stop // dim], device=ids.device)
+        cuts = torch.searchsorted(ids, bounds).tolist()  # (the row counts travel in the request)
+        pflat = _flat(p)
+        for k, c in enumerate(per):
+            lo, hi = cuts[k], cuts[k + 1]
+            r = hi - lo
+            rows = (c.stop - c.start) // dim
+            stage = self._staging.get(c.key)
+            if stage is None:
+                stage = torch.zeros(C.rows_slot_bytes(rows, dim, fmt), dtype=torch.uint8, device=p.device)
+                self._staging[c.key] = stage
+            nbytes = C.rows_slot_bytes(r, dim, fmt)
+            if r:
+                ids_w = (r + 3) // 4 * 4
+                stage[:4 * r].view(torch.int32).copy_(ids[lo:hi] - c.start // dim)
+                stage[4 * r:4 * ids_w].zero_()
+                body = stage[4 * ids_w:nbytes]
+                v = vals[lo:hi].reshape(-1)
+                if fmt == C.GRAD_FP8BLOCK:
+                    C.copy_codec(body, v.contiguous(), C.CODEC_F32_TO_FP8BLOCK, 1.0)
+                else:
+                    body.view(torch.bfloat16).copy_(v)
+                payload = stage[:nbytes]
+            else:
+                payload = stage[:16].zero_()  # a worker whose batch touched no row of this chunk still takes part
+            self._pending.append(self.kv.push(c.key, payload, cmd=C.CMD_GRAD_ROWS, codec=C.CODEC_RAW,
+                                              option=(r << 2) | fmt, slot_bytes=stage.numel()))
+            self._pending.append(self.kv.pull(c.key, pflat[c.start:c.stop], symm_offset=self._symm(c)))
+            self.stats.pushes += 1
+            self.stats.pulls += 1
+            self.stats.push_bytes_wire += payload.numel()
+            self.stats.pull_bytes += (c.stop - c.start) * 2
+
     def _push_pull_now(self, i: int, g: torch.Tensor):
+        if self.chunks[i] and self.chunks[i][0].dim:
+            self._push_rows(i, g)
+            return
         p = self.params[i].data
         if p.is_contiguous():
             if not g.is_contiguous():

@@ -320,3 +320,122 @@ extern "C" int ps_host_update(const ps_update_args* a, const ps_opt_params* o) {
   });
   return 0;
 }
+
+extern "C" size_t ps_rows_scratch_bytes(size_t rows, int max_grads) {
+  return sizeof(ps_rows_scratch_hdr) + rows * 4 * (2 + static_cast<size_t>(max_grads));
+}
+
+namespace {
+template <int FMT>
+void UpdateRows(const ps_update_rows_args& a, const ps_opt_params& opt, const uint32_t* pos,
+                const uint32_t* list, size_t r0, size_t r1) {
+  const size_t D = static_cast<size_t>(a.dim);
+  const float* e4m3 = E4m3Table();
+  const bool adam = opt.optimizer == PS_OPT_ADAMW;
+  const float inv_bc1 = adam ? 1.f / opt.bias_corr1 : 1.f, inv_bc2 = adam ? 1.f / opt.bias_corr2 : 1.f;
+  std::vector<float> g(D);
+  for (size_t r = r0; r < r1; ++r) {
+    const size_t id = list[r];
+    std::fill(g.begin(), g.end(), 0.f);
+    for (int w = 0; w < a.num_grads; ++w) {  // fixed slot order, as on the GPU
+      const uint32_t s = pos[static_cast<size_t>(w) * a.rows + id];
+      if (s == 0) continue;
+      const size_t i = ~s;
+      const unsigned char* vals = static_cast<const unsigned char*>(a.grads[w]) +
+                                  (static_cast<size_t>(a.num_rows[w]) + 3) / 4 * 16;
+      if (FMT == PS_GRAD_BF16) {
+        const uint16_t* q = reinterpret_cast<const uint16_t*>(vals) + i * D;
+        for (size_t j = 0; j < D; ++j) g[j] += Bf16ToF32(q[j]);
+      } else if (FMT == PS_GRAD_FP8BLOCK) {
+        const unsigned char* q = vals + i * D;
+        const unsigned char* sc = vals + static_cast<size_t>(a.num_rows[w]) * D + i * D / 32;
+        for (size_t j = 0; j < D; ++j) g[j] += e4m3[q[j]] * Exp2FromE8m0(sc[j >> 5]);
+      } else {
+        const float* q = reinterpret_cast<const float*>(vals) + i * D;
+        for (size_t j = 0; j < D; ++j) g[j] += q[j];
+      }
+    }
+    float* p = a.master + id * D;
+    float* m = a.m + id * D;
+    float* v = adam ? a.v + id * D : nullptr;
+    for (size_t j = 0; j < D; ++j) {
+      const float gj = g[j] * opt.grad_scale;
+      float pn;
+      if (adam) {
+        const float mj = opt.beta1 * m[j] + (1.f - opt.beta1) * gj;
+        const float vj = opt.beta2 * v[j] + (1.f - opt.beta2) * gj * gj;
+        const float denom = std::sqrt(vj * inv_bc2) + opt.eps;
+        pn = p[j] - opt.lr * ((mj * inv_bc1) / denom + opt.weight_decay * p[j]);
+        m[j] = mj;
+        v[j] = vj;
+      } else {
+        const float gw = gj + opt.weight_decay * p[j];
+        const float mj = opt.beta1 * m[j] + gw;
+        pn = p[j] - opt.lr * mj;
+        m[j] = mj;
+      }
+      p[j] = pn;
+    }
+    for (int k = 0; k < a.num_outs; ++k) {
+      if (a.out_f32) {
+        memcpy(static_cast<float*>(a.outs[k]) + id * D, p, D * 4);
+      } else {
+        uint16_t* out = static_cast<uint16_t*>(a.outs[k]) + id * D;
+        for (size_t j = 0; j < D; ++j) out[j] = F32ToBf16(p[j]);
+      }
+    }
+  }
+}
+}  // namespace
+
+extern "C" int ps_host_update_rows(const ps_update_rows_args* args, const ps_opt_params* o) {
+  const ps_update_rows_args a = *args;
+  if (a.num_grads < 1 || a.num_grads > PS_MAX_FANIN) return 1;
+  if (a.num_outs < 0 || a.num_outs > PS_MAX_FANOUT) return 1;
+  if (a.dim <= 0 || a.dim % 8 != 0 || a.rows > 0xffffffffull) return 1;
+  const int fmt = a.grad_format;
+  if (fmt != PS_GRAD_BF16 && fmt != PS_GRAD_FP8BLOCK && fmt != PS_GRAD_F32) return 1;
+  if (fmt == PS_GRAD_FP8BLOCK && a.dim % 32 != 0) return 1;
+  size_t total = 0;
+  for (int w = 0; w < a.num_grads; ++w) total += a.num_rows[w];
+  if (total == 0) return 0;
+  // the same scratch and the same marking rules as k_rows_mark (update_rows_kernels.cu)
+  ps_rows_scratch_hdr* hdr = static_cast<ps_rows_scratch_hdr*>(a.scratch);
+  uint32_t* touched = reinterpret_cast<uint32_t*>(hdr + 1);
+  uint32_t* list = touched + a.rows;
+  uint32_t* pos = list + a.rows;
+  uint32_t count = 0;
+  for (int w = 0; w < a.num_grads; ++w) {
+    const uint32_t* ids = static_cast<const uint32_t*>(a.grads[w]);
+    for (uint32_t i = 0; i < a.num_rows[w]; ++i) {
+      const uint32_t id = ids[i];
+      if (id >= a.rows) {
+        ++hdr->bad;
+        continue;
+      }
+      uint32_t& s = pos[static_cast<size_t>(w) * a.rows + id];
+      if (s != 0) {  // a repeated id: its first occurrence stays
+        ++hdr->bad;
+        continue;
+      }
+      s = ~i;
+      if (!touched[id]) {
+        touched[id] = 1;
+        list[count++] = id;
+      }
+    }
+  }
+  const ps_opt_params opt = *o;
+  ParallelFor(static_cast<size_t>(count) * a.dim, a.dim, [&](size_t e0, size_t e1) {
+    const size_t r0 = e0 / a.dim, r1 = e1 / a.dim;
+    if (fmt == PS_GRAD_BF16) UpdateRows<PS_GRAD_BF16>(a, opt, pos, list, r0, r1);
+    else if (fmt == PS_GRAD_FP8BLOCK) UpdateRows<PS_GRAD_FP8BLOCK>(a, opt, pos, list, r0, r1);
+    else UpdateRows<PS_GRAD_F32>(a, opt, pos, list, r0, r1);
+  });
+  for (uint32_t r = 0; r < count; ++r) {
+    const uint32_t id = list[r];
+    touched[id] = 0;
+    for (int w = 0; w < a.num_grads; ++w) pos[static_cast<size_t>(w) * a.rows + id] = 0;
+  }
+  return 0;
+}

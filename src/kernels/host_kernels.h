@@ -25,6 +25,8 @@ int ps_host_sum(float* out_f32, const void* const* grads, int num_grads, int gra
                 float scale, int accumulate);
 /*! \brief fused dequant + W-way sum + AdamW / SGD + bf16 (or fp32) fan-out; mc_out is ignored */
 int ps_host_update(const ps_update_args* args, const ps_opt_params* opt);
+/*! \brief row-sparse twin of ps_launch_update_rows: same slot layout, scratch and bad-id counting */
+int ps_host_update_rows(const ps_update_rows_args* args, const ps_opt_params* opt);
 
 #ifdef __cplusplus
 }

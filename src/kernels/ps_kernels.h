@@ -13,6 +13,8 @@
  *                       fp32 master / moments, and emit bf16 parameters to up to
  *                       8 destinations at once (local shard copy + every worker's
  *                       parameter buffer, i.e. update fused with the pull reply).
+ *   ps_launch_update_rows  the same for a row-sparse shard (embedding table): only the rows
+ *                       some worker pushed are summed, stepped and fanned out.
  *   ps_launch_sum       plain W-way dequantising reduction (KVServer default handle).
  * All take a cudaStream_t and never synchronise. No cuBLAS/NCCL anywhere.
  */
@@ -164,6 +166,56 @@ typedef struct {
  */
 int ps_launch_update(const ps_update_args* args, const ps_opt_params* opt, int max_ctas,
                      ps_stream_t stream);
+
+/*!
+ * \brief one round of a ROW-SPARSE shard of rows x dim fp32 elements (an embedding table).
+ *        Slot w holds num_rows[w] = R_w unique local row ids and their gradient rows:
+ *            [u32 ids, R_w entries, zero-padded to a multiple of 4][values]
+ *            values: PS_GRAD_F32  R_w*dim f32 | PS_GRAD_BF16  R_w*dim bf16 |
+ *                    PS_GRAD_FP8BLOCK  [R_w*dim e4m3][R_w*dim/32 e8m0]   (dim % 32 == 0)
+ *        The contributions to each row of the union are summed in slot order (w = 0..W-1), the
+ *        optimizer step runs on those rows only ("lazy": untouched rows keep master, m and v bit
+ *        for bit and get no weight decay), and the new rows are stored at their row offsets into
+ *        every outs[k]; nothing else of a destination is written. R_w = 0 is legal.
+ *        An id >= rows, or an id repeated within one slot (its first occurrence is used), is
+ *        skipped and counted in the scratch header's `bad`.
+ */
+typedef struct {
+  size_t rows;                         // rows in the shard
+  int dim;                             // D: elements per row, a multiple of 8
+  int num_grads;                       // W, 1..PS_MAX_FANIN
+  int grad_format;                     // PS_GRAD_F32 / PS_GRAD_BF16 / PS_GRAD_FP8BLOCK
+  const void* grads[PS_MAX_FANIN];     // W slots in the layout above
+  uint32_t num_rows[PS_MAX_FANIN];     // R_w
+  float* master;                       // rows x dim fp32 (in/out)
+  float* m;
+  float* v;                            // AdamW only
+  int num_outs;                        // destinations, each rows x dim
+  void* outs[PS_MAX_FANOUT];
+  int out_f32;                         // outs[] receive fp32 instead of bf16
+  /* ps_rows_scratch_bytes(rows, >= W) bytes, zero-filled once when allocated: every launch
+   * leaves it zeroed again except for the header's `bad`, so it is kept between rounds */
+  void* scratch;
+} ps_update_rows_args;
+
+/*! \brief head of the row-sparse scratch; then u32 touched[rows], list[rows], slot_of[W][rows] */
+typedef struct {
+  uint32_t count;            // rows in the union of the current launch
+  uint32_t done;             // CTAs finished (the last one resets count and done)
+  unsigned long long bad;    // ids skipped since the scratch was allocated (never reset)
+} ps_rows_scratch_hdr;
+
+size_t ps_rows_scratch_bytes(size_t rows, int max_grads);
+
+/*!
+ * \brief row-sparse fused update: marks the union on the device, then one grid sized to the GPU
+ *        walks it (gather-sum, optimizer, scatter). No host synchronisation.
+ * \return cudaErrorInvalidValue for bad counts, formats or dim; cudaErrorMisalignedAddress, before
+ *         anything is launched, unless master, m, v (AdamW), every grads[w] and every outs[k] are
+ *         16-byte aligned
+ */
+int ps_launch_update_rows(const ps_update_rows_args* args, const ps_opt_params* opt, int max_ctas,
+                          ps_stream_t stream);
 
 /*! \brief out_f32[i] (+)= sum_w decode(grads[w])[i] * scale */
 int ps_launch_sum(float* out_f32, const void* const* grads, int num_grads, int grad_format,

@@ -19,8 +19,6 @@
  * Each thread-iteration handles 8 elements: 16-byte loads for bf16 grads, 8-byte
  * for fp8, 2 x 16-byte for each fp32 state array, 16-byte bf16 stores.
  */
-#include <cuda_bf16.h>
-#include <cuda_fp8.h>
 #include <cuda_runtime.h>
 
 #include <atomic>
@@ -29,6 +27,7 @@
 #include <cstdlib>
 
 #include "kernels/ps_kernels.h"
+#include "kernels/update_math.cuh"
 
 namespace ps_kernels_internal {
 void CountLaunch(int n);
@@ -54,37 +53,6 @@ struct UpdateDev {
   int body_outs;    // unicast outputs written in the vector body
 };
 
-__device__ __forceinline__ int4 ldg16(const void* p) {
-  int4 r;
-  asm volatile("ld.global.nc.L1::no_allocate.v4.s32 {%0,%1,%2,%3}, [%4];"
-               : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w)
-               : "l"(p));
-  return r;
-}
-__device__ __forceinline__ uint2 ldg8(const void* p) {
-  uint2 r;
-  asm volatile("ld.global.nc.L1::no_allocate.v2.u32 {%0,%1}, [%2];"
-               : "=r"(r.x), "=r"(r.y)
-               : "l"(p));
-  return r;
-}
-__device__ __forceinline__ float4 ldf4(const float* p) {
-  float4 r;
-  asm volatile("ld.global.L1::no_allocate.v4.f32 {%0,%1,%2,%3}, [%4];"
-               : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w)
-               : "l"(p));
-  return r;
-}
-__device__ __forceinline__ void stf4(float* p, const float4& v) {
-  asm volatile("st.global.L1::no_allocate.v4.f32 [%0], {%1,%2,%3,%4};" ::"l"(p), "f"(v.x),
-               "f"(v.y), "f"(v.z), "f"(v.w)
-               : "memory");
-}
-__device__ __forceinline__ void st16(void* p, const int4& v) {
-  asm volatile("st.global.L1::no_allocate.v4.s32 [%0], {%1,%2,%3,%4};" ::"l"(p), "r"(v.x),
-               "r"(v.y), "r"(v.z), "r"(v.w)
-               : "memory");
-}
 /*! one store, replicated by the NVSwitch to every GPU bound to the multicast object */
 __device__ __forceinline__ void multimem_st16(void* p, const int4& v) {
   asm volatile("multimem.st.relaxed.sys.global.v4.f32 [%0], {%1,%2,%3,%4};" ::"l"(p),
@@ -109,27 +77,6 @@ __device__ __forceinline__ uint32_t multimem_ld_reduce4(const void* p) {
                : "memory");
   return r;
 }
-__device__ __forceinline__ float2 bf2(uint32_t u) {
-  __nv_bfloat162 t = *reinterpret_cast<__nv_bfloat162*>(&u);
-  return __bfloat1622float2(t);
-}
-__device__ __forceinline__ uint32_t pk(float lo, float hi) {
-  __nv_bfloat162 t = __floats2bfloat162_rn(lo, hi);
-  return *reinterpret_cast<uint32_t*>(&t);
-}
-__device__ __forceinline__ float e8m0(uint32_t biased) {
-  const int be = max(1, min(254, static_cast<int>(biased)));
-  return __uint_as_float(static_cast<uint32_t>(be) << 23);
-}
-__device__ __forceinline__ void fp8x4_to_f32(uint32_t q, float s, float* out) {
-  const __half2_raw lo = __nv_cvt_fp8x2_to_halfraw2(static_cast<__nv_fp8x2_storage_t>(q & 0xffffu),
-                                                    __NV_E4M3);
-  const __half2_raw hi = __nv_cvt_fp8x2_to_halfraw2(static_cast<__nv_fp8x2_storage_t>(q >> 16),
-                                                    __NV_E4M3);
-  const float2 a = __half22float2(__half2(lo)), b = __half22float2(__half2(hi));
-  out[0] = a.x * s; out[1] = a.y * s; out[2] = b.x * s; out[3] = b.y * s;
-}
-
 /*! \brief sum of 8 consecutive gradient elements starting at 8*i over all W slots */
 template <int FMT>
 __device__ __forceinline__ void gather_grads(const UpdateDev& a, size_t i, float* g) {
@@ -193,35 +140,6 @@ __device__ __forceinline__ float gather_one(const UpdateDev& a, size_t e) {
     }
   }
   return g;
-}
-
-/*! single-instruction MUFU.SQRT (<= 1 ulp-ish); the IEEE sqrtf expands to ~10 instructions */
-__device__ __forceinline__ float fast_sqrt(float x) {
-  float r;
-  asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
-  return r;
-}
-
-/*!
- * o.bias_corr1 / o.bias_corr2 hold the RECIPROCALS 1/(1-beta^t) here (ps_launch_update
- * inverts them on the host) so the per-element math is FMA + one MUFU.SQRT + one MUFU.RCP:
- * the kernel must stay memory-bound, and the IEEE div/sqrt sequences cost ~170 issue slots
- * per element, right at the instruction roofline for 28 B/element at 6.5 TB/s.
- */
-template <int OPT>
-__device__ __forceinline__ void step(float& p, float& m, float& v, float g,
-                                     const ps_opt_params& o) {
-  if (OPT == PS_OPT_ADAMW) {
-    m = fmaf(o.beta1, m, (1.f - o.beta1) * g);
-    v = fmaf(o.beta2, v, (1.f - o.beta2) * g * g);
-    const float denom = fast_sqrt(v * o.bias_corr2) + o.eps;
-    const float upd = __fdividef(m * o.bias_corr1, denom);
-    p = p - o.lr * fmaf(o.weight_decay, p, upd);
-  } else {
-    g += o.weight_decay * p;
-    m = o.beta1 * m + g;
-    p = p - o.lr * m;
-  }
 }
 
 template <int FMT, int OPT, bool OUT_F32>

@@ -36,6 +36,7 @@ class GpuServer::Backend {
   virtual void Free(void* p) = 0;
   virtual void Decode(float* dst, const void* wire, size_t n, int fmt) = 0;
   virtual void Update(const ps_update_args& a, const ps_opt_params& o, int max_ctas) = 0;
+  virtual void UpdateRows(const ps_update_rows_args& a, const ps_opt_params& o, int max_ctas) = 0;
   virtual void Copy(void* dst, const void* src, size_t n_src_bytes, int codec, float scale,
                     int max_ctas) = 0;
   /*! \brief synchronous transfers between backend memory and host memory */
@@ -61,6 +62,9 @@ class HostBackend : public GpuServer::Backend {
   }
   void Update(const ps_update_args& a, const ps_opt_params& o, int /*max_ctas*/) override {
     CHECK_EQ(ps_host_update(&a, &o), 0) << "unsupported gradient format " << a.grad_format;
+  }
+  void UpdateRows(const ps_update_rows_args& a, const ps_opt_params& o, int /*max_ctas*/) override {
+    CHECK_EQ(ps_host_update_rows(&a, &o), 0) << "bad row-sparse update (format " << a.grad_format << ")";
   }
   void Copy(void* dst, const void* src, size_t n, int codec, float scale, int /*max_ctas*/) override {
     CHECK_EQ(ps_host_copy(dst, src, n, codec, scale), 0);
@@ -105,6 +109,9 @@ class CudaBackend : public GpuServer::Backend {
   }
   void Update(const ps_update_args& a, const ps_opt_params& o, int max_ctas) override {
     CHECK_EQ(ps_launch_update(&a, &o, max_ctas, ps_stream()), 0);
+  }
+  void UpdateRows(const ps_update_rows_args& a, const ps_opt_params& o, int max_ctas) override {
+    CHECK_EQ(ps_launch_update_rows(&a, &o, max_ctas, ps_stream()), 0);
   }
   void Copy(void* dst, const void* src, size_t n, int codec, float scale, int max_ctas) override {
     CHECK_EQ(ps_launch_copy(dst, src, n, codec, scale, max_ctas, ps_stream()), 0);
@@ -186,6 +193,7 @@ GpuServer::~GpuServer() {
     be_->Free(kv.second.master);
     be_->Free(kv.second.m);
     be_->Free(kv.second.v);
+    if (kv.second.scratch) be_->Free(kv.second.scratch);
     for (void* p : kv.second.staged) {
       if (p) be_->Free(p);
     }
@@ -227,8 +235,60 @@ size_t GpuServer::num_keys() {
 size_t GpuServer::state_bytes() {
   std::lock_guard<std::mutex> lk(mu_);
   size_t b = 0;
-  for (auto& kv : shards_) b += kv.second.n * 12;
+  for (auto& kv : shards_) {
+    b += kv.second.n * 12;
+    if (kv.second.dim) b += ps_rows_scratch_bytes(kv.second.n / kv.second.dim, cfg_.num_workers);
+  }
   return b;
+}
+
+uint64_t GpuServer::num_bad_rows() {
+  std::lock_guard<std::mutex> lk(mu_);
+  be_->Bind();
+  uint64_t bad = 0;
+  for (auto& kv : shards_) {
+    if (!kv.second.scratch) continue;
+    ps_rows_scratch_hdr h;
+    be_->Download(&h, kv.second.scratch, sizeof(h));
+    bad += h.bad;
+  }
+  return bad;
+}
+
+void GpuServer::MakeRowSparse(Shard* s, int dim) {
+  CHECK_GT(dim, 0) << "a row-sparse shard needs its row width in option bits 8..30";
+  CHECK_EQ(dim % 8, 0) << "row-sparse shard: the row width " << dim
+                       << " is not a multiple of 8 (rows move as 16-byte vectors)";
+  CHECK_EQ(s->n % static_cast<size_t>(dim), (size_t)0)
+      << "row-sparse shard: " << s->n << " elements are not a whole number of rows of " << dim;
+  CHECK_LE(s->n / dim, (size_t)0xffffffffu) << "row-sparse shard: row ids are 32-bit";
+  s->dim = dim;
+  s->scratch = be_->Alloc(ps_rows_scratch_bytes(s->n / dim, cfg_.num_workers));  // zero-filled
+  s->num_rows.assign(cfg_.num_workers, 0);
+}
+
+void GpuServer::RunUpdate(Shard* s, const ps_update_args& a, const ps_opt_params& o, int first_rank) {
+  if (!s->dim) {
+    be_->Update(a, o, cfg_.max_ctas);
+    return;
+  }
+  ps_update_rows_args r;
+  memset(&r, 0, sizeof(r));
+  r.rows = s->n / s->dim;
+  r.dim = s->dim;
+  r.num_grads = a.num_grads;
+  r.grad_format = a.grad_format;
+  for (int w = 0; w < a.num_grads; ++w) {
+    r.grads[w] = a.grads[w];
+    r.num_rows[w] = s->num_rows[first_rank + w];
+  }
+  r.master = a.master;
+  r.m = a.m;
+  r.v = a.v;
+  r.num_outs = a.num_outs;  // unicast only: row shards never use the multicast fan-out
+  for (int k = 0; k < a.num_outs; ++k) r.outs[k] = a.outs[k];
+  r.scratch = s->scratch;
+  be_->UpdateRows(r, o, cfg_.max_ctas);
 }
 
 size_t GpuServer::ElemsOf(const KVMeta& req) {
@@ -289,6 +349,17 @@ void GpuServer::Handle(const KVMeta& req, const KVPairs<char>& data, KVServer<ch
     server_->Response(req);
     return;
   }
+  if (req.push && req.cmd == kCmdGradRows) {
+    // the payload size varies with the rows pushed: the shard must exist (its init push came first)
+    auto it = shards_.find(key);
+    CHECK(it != shards_.end()) << "row-sparse gradient (kCmdGradRows) for key " << key
+                               << ", which was never initialised";
+    CHECK(!req.pull) << "kCmdGradRows is pushed, then pulled";
+    Shard* s = &it->second;
+    HandleGrad(s, req, data);
+    MaybeRunRound(key, s);
+    return;
+  }
   if (req.push) {
     Shard* s = GetShard(key, ElemsOf(req));
     if (req.cmd == kCmdInitBf16 || req.cmd == kCmdInitF32) {
@@ -333,6 +404,7 @@ void GpuServer::HandleInit(Shard* s, const KVMeta& req, const KVPairs<char>& dat
     }
     s->initialized = true;
     s->no_weight_decay = (req.option & kInitNoWeightDecay) != 0;
+    if (req.option & kInitRowSparse) MakeRowSparse(s, (req.option >> 8) & 0x7fffff);
   }
   server_->Response(req);
 }
@@ -342,8 +414,28 @@ void GpuServer::HandleGrad(Shard* s, const KVMeta& req, const KVPairs<char>& dat
   CHECK_LT(rank, cfg_.num_workers);
   CHECK(!s->pushed[rank]) << "worker " << rank << " pushed key " << req.key
                           << " twice in one round";
-  int fmt;
+  int fmt = PS_GRAD_BF16;
   const void* slot;
+  if (req.cmd == kCmdGradRows) {
+    CHECK(s->dim > 0) << "key " << req.key << " is a dense shard: it takes kCmdGrad pushes, not kCmdGradRows";
+    CHECK_EQ(req.codec, (int)kCodecRaw) << "kCmdGradRows payloads are encoded by the worker (codec raw)";
+    CHECK_NE(req.mem.region, kSymmetricRegion) << "row-sparse gradients are not reduced in the switch";
+    const int row_format = req.option & 3;
+    const size_t R = static_cast<uint32_t>(req.option) >> 2;
+    CHECK(row_format == PS_GRAD_F32 || row_format == PS_GRAD_BF16 || row_format == PS_GRAD_FP8BLOCK)
+        << "kCmdGradRows: unknown row format " << row_format;
+    CHECK(row_format != PS_GRAD_FP8BLOCK || s->dim % 32 == 0)
+        << "kCmdGradRows: fp8 rows need a row width that is a multiple of 32, the shard has " << s->dim;
+    const size_t e = R * s->dim;
+    const size_t need = (R + 3) / 4 * 16 +
+                        (row_format == PS_GRAD_F32 ? 4 * e : row_format == PS_GRAD_BF16 ? 2 * e : e + e / 32);
+    CHECK_GE(data.vals.size(), need) << "kCmdGradRows: " << R << " rows need " << need << " bytes";
+    s->num_rows[rank] = static_cast<uint32_t>(R);
+    fmt = row_format;
+  } else {
+    CHECK_EQ(s->dim, 0) << "key " << req.key
+                        << " is a row-sparse shard: it takes kCmdGradRows pushes only";
+  }
   if (req.mem.region == kSymmetricRegion) {
     // staged in the worker's symmetric gradient buffer: read later through the multicast address
     CHECK(mc_grad_base_ != nullptr) << "symmetric push but SetSymmetricGrads was never called";
@@ -377,7 +469,7 @@ void GpuServer::HandleGrad(Shard* s, const KVMeta& req, const KVPairs<char>& dat
       CHECK(!data.vals.on_gpu()) << "this server keeps its shards in host memory";
       s->slot_refs[rank] = data.vals;  // a two-sided payload lives in a pooled receive buffer
     }
-    fmt = FormatOf(req, cfg_.raw_grad_format);
+    if (req.cmd != kCmdGradRows) fmt = FormatOf(req, cfg_.raw_grad_format);
   }
   if (s->num_pushed == 0) s->grad_format = fmt;
   CHECK_EQ(s->grad_format, fmt) << "workers disagree on the gradient wire format";
@@ -446,7 +538,7 @@ void GpuServer::ApplyOnArrival(Shard* s, int rank) {
     o.bias_corr1 = 1.f - std::pow(o.beta1, static_cast<float>(s->step));
     o.bias_corr2 = 1.f - std::pow(o.beta2, static_cast<float>(s->step));
   }
-  be_->Update(a, o, cfg_.max_ctas);
+  RunUpdate(s, a, o, rank);
   ++updates_;
   // the slot may be overwritten by this worker's next push as soon as it is acked: on the
   // device the ack is sent behind the update on the same stream, on the host Update is synchronous
@@ -477,7 +569,8 @@ void GpuServer::MaybeRunRound(Key key, Shard* s) {
   a.v = s->v;
   a.num_outs = 0;  // no server-side bf16 copy: late pulls are cast from the fp32 master on demand
   std::vector<char> placed(s->waiting_pulls.size(), 0);
-  bool all_symmetric = mc_base_ != nullptr && static_cast<int>(s->waiting_pulls.size()) == W;
+  // (a row shard writes its touched rows into every placed destination with unicast stores)
+  bool all_symmetric = mc_base_ != nullptr && static_cast<int>(s->waiting_pulls.size()) == W && !s->dim;
   for (size_t i = 0; i < s->waiting_pulls.size(); ++i) {
     const KVMeta& pull = s->waiting_pulls[i];
     void* dst = WorkerDest(pull);
@@ -504,7 +597,7 @@ void GpuServer::MaybeRunRound(Key key, Shard* s) {
     o.bias_corr1 = 1.f - std::pow(o.beta1, static_cast<float>(s->step));
     o.bias_corr2 = 1.f - std::pow(o.beta2, static_cast<float>(s->step));
   }
-  be_->Update(a, o, cfg_.max_ctas);
+  RunUpdate(s, a, o, 0);
   ++updates_;
   if (a.num_outs > 0) ++fused_;
 
@@ -615,7 +708,9 @@ bool GpuServer::SaveCheckpoint(const std::string& path) {
   std::vector<float> buf;
   for (auto& kv : shards_) {
     const Shard& s = kv.second;
-    CkptEntry e{kv.first, s.n, s.step, (s.initialized ? 1 : 0) | (s.no_weight_decay ? 2 : 0)};
+    // bit 0 initialized, bit 1 no weight decay, bit 2 row-sparse with the row width in bits 8..30
+    CkptEntry e{kv.first, s.n, s.step,
+                (s.initialized ? 1 : 0) | (s.no_weight_decay ? 2 : 0) | (s.dim ? 4 | (s.dim << 8) : 0)};
     ok = ok && fwrite(&e, sizeof(e), 1, f) == 1;
     buf.resize(s.n);
     for (float* src : {s.master, s.m, s.v}) {
@@ -643,6 +738,11 @@ bool GpuServer::LoadCheckpoint(const std::string& path) {
     s->step = e.step;
     s->initialized = (e.initialized & 1) != 0;
     s->no_weight_decay = (e.initialized & 2) != 0;
+    const int dim = (e.initialized & 4) ? (e.initialized >> 8) & 0x7fffff : 0;
+    if (dim != s->dim) {
+      CHECK_EQ(s->dim, 0) << "checkpoint: key " << e.key << " has rows of " << dim << ", this server " << s->dim;
+      MakeRowSparse(s, dim);  // (its scratch is not saved: a fresh one is empty)
+    }
     buf.resize(e.n);
     for (float* dst : {s->master, s->m, s->v}) {
       ok = ok && fread(buf.data(), 4, e.n, f) == e.n;

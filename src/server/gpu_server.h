@@ -43,6 +43,9 @@ namespace ps {
 /*! \brief KVMeta::option bits of an initial-value push (per-shard optimizer settings) */
 enum GpuServerInitOption : int {
   kInitNoWeightDecay = 1,  // norms, biases, embeddings: exclude this shard from weight decay
+  /* a row-sparse shard (embedding table): option = flags | (D << 8), D = row width in elements
+   * (a multiple of 8, D < 2^23); gradients then arrive as kCmdGradRows pushes */
+  kInitRowSparse = 2,
 };
 
 /*! \brief `cmd` values understood by GpuServer */
@@ -51,6 +54,9 @@ enum GpuServerCmd : int {
   kCmdInitBf16 = 101,  // push: initial parameter values, bf16 (first writer wins)
   kCmdInitF32 = 102,   // push: initial parameter values, fp32
   kCmdSetLr = 103,     // push: one fp32 value = new learning rate of this server (any key it owns)
+  /* push, codec kCodecRaw, option = (R << 2) | PS_GRAD_F32 / PS_GRAD_BF16 / PS_GRAD_FP8BLOCK:
+   * R rows of a row-sparse shard, laid out as ps_update_rows_args describes. R may be 0. */
+  kCmdGradRows = 104,
 };
 
 struct GpuServerConfig {
@@ -115,8 +121,11 @@ class GpuServer {
   /*! \brief update kernels whose destinations included worker buffers (fused pull replies) */
   uint64_t num_fused_fanouts() const { return fused_.load(); }
   size_t num_keys();
-  /*! \brief bytes of HBM held by parameter + optimizer state */
+  /*! \brief bytes of HBM held by parameter + optimizer state (and the scratch of row-sparse shards) */
   size_t state_bytes();
+  /*! \brief row ids skipped by row-sparse updates (>= rows, or repeated in one push), summed over
+   *         shards. Synchronous device read: for tests and diagnostics */
+  uint64_t num_bad_rows();
 
   /*! \brief dump / restore every shard this server owns (fp32 master, m, v, step) */
   bool SaveCheckpoint(const std::string& path);
@@ -141,6 +150,9 @@ class GpuServer {
     bool no_weight_decay = false;
     int step = 0;
     int grad_format = PS_GRAD_BF16;
+    int dim = 0;                         // row-sparse shard: row width; 0 = dense
+    void* scratch = nullptr;             // row-sparse shard: ps_rows_scratch_bytes(n / dim, W)
+    std::vector<uint32_t> num_rows;      // row-sparse shard: rows pushed per worker rank this round
     std::vector<const void*> slots;      // per worker rank: landing slot of this round
     std::vector<SArray<char>> slot_refs; // host shards: keeps a two-sided payload alive until the round runs
     std::vector<void*> staged;           // device shards: per rank, where a gradient that arrived in HOST memory
@@ -157,6 +169,8 @@ class GpuServer {
   void MaybeRunRound(Key key, Shard* s);
   void ApplyOnArrival(Shard* s, int rank);
   void ServePullFromLocal(Key key, Shard* s, const KVMeta& req);
+  void MakeRowSparse(Shard* s, int dim);
+  void RunUpdate(Shard* s, const ps_update_args& a, const ps_opt_params& o, int first_rank);
   Shard* GetShard(Key key, size_t n);
   void* WorkerDest(const KVMeta& pull);
   static size_t ElemsOf(const KVMeta& req);

@@ -218,6 +218,7 @@ class OneSidedVan : public TcpVan {
     out->emplace_back("onesided_bytes", copy_bytes_.load());
     out->emplace_back("gated_frames", gated_frames_.load());
     out->emplace_back("staged_copies", staged_copies_.load());
+    out->emplace_back("push_slot_rendezvous", slot_rendezvous_.load());
     out->emplace_back("recv_thread_sleeps", num_blocking_waits());
     out->emplace_back("deferred_sends", num_deferred_sends());
     out->emplace_back("engine_launches", launches);
@@ -534,7 +535,8 @@ class OneSidedVan : public TcpVan {
       slot.region = kSymmetricRegion;
       slot.offset = msg.meta.mem.offset;
     } else {
-      slot = AcquirePushSlot(recver, msg.meta.key, wire, vals.dst_device_type_ == GPU ? vals.dst_device_id_ : -1);
+      slot = AcquirePushSlot(recver, msg.meta.key, wire, vals.dst_device_type_ == GPU ? vals.dst_device_id_ : -1,
+                             msg.slot_bytes);
     }
     MemDomain::CopyItem item;
     item.dst = slot.ptr;
@@ -565,15 +567,20 @@ class OneSidedVan : public TcpVan {
     return Submit(desc, &item, false, vals) + static_cast<int>(std::min<uint64_t>(wire, 0x3fffffff));
   }
 
-  /*! \brief landing slot at `recver` for `key`; rendezvous on first use or growth */
-  Slot AcquirePushSlot(int recver, uint64_t key, uint64_t bytes, int dst_device = -1) {
+  /*!
+   * \brief landing slot at `recver` for `key`; rendezvous on first use or growth. With `slot_bytes`
+   *        (SendOpts::slot_bytes) the slot is requested at that capacity and kept while pushes fit.
+   */
+  Slot AcquirePushSlot(int recver, uint64_t key, uint64_t bytes, int dst_device = -1, uint64_t slot_bytes = 0) {
     std::unique_lock<SpinMutex> lk(rv_mu_);
     const PeerKey pk(recver, key);
     auto it = push_slots_.find(pk);
     if (it != push_slots_.end() && it->second.capacity >= bytes &&
-        !Oversized(it->second.capacity, bytes)) {
+        (slot_bytes != 0 || !Oversized(it->second.capacity, bytes))) {
       return it->second;
     }
+    bytes = std::max(bytes, slot_bytes);
+    ++slot_rendezvous_;
     push_slots_.erase(pk);  // too small, or far too large (e.g. bf16 init, then fp8 gradients)
     lk.unlock();
     Message req;
@@ -1045,6 +1052,7 @@ class OneSidedVan : public TcpVan {
   std::atomic<int> staged_pulls_pending_{0};
   std::atomic<int> registered_count_{0};  // size of registered_slots_ (checked without the lock per frame)
   std::atomic<uint64_t> staged_copies_{0};
+  std::atomic<uint64_t> slot_rendezvous_{0};  // ADDR_REQUESTs sent for push landing slots
 
   SpinMutex cq_mu_;
   std::condition_variable_any cq_cv_;
